@@ -14,6 +14,8 @@ its predecessor.  Mkeypoints/s = keypoints extracted-and-matched / time.
           step's frames from pinned memory and D2H of keypoints/descriptors inside the timed region.
 
 `--impl reference` times the CPU oracle port of the reference path (oracle/) on the host cores.
+`--dump-outputs DIR` writes what the value path returned in the last timed step, for a fixed sample of the step's frames, as
+DIR/<name>.npy (float32); the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 PyTorch is used only for plumbing: device buffers, pinned host memory, torch.distributed.
 """
 import argparse
@@ -34,6 +36,7 @@ FX = FY = 1000.0
 CX, CY = W / 2.0, H / 2.0
 DEPTH = 5.0
 MATCH_TH = 15.0  # Tracking.cc:565
+DUMP_FRAMES = 32  # frames of the last step written by --dump-outputs: 32 x 2000 keypoints x 40 floats = 10 MB
 METRIC = "Mkeypoints/s extract+match"
 
 
@@ -383,7 +386,11 @@ def main():
                          "SearchForInitialization); dbsweep = configs[4] (sharded keyframe-database sweep): the last two print their own line")
     ap.add_argument("--slots", type=int, default=8, help="rig8: time steps per exchange")
     ap.add_argument("--groups", type=int, default=10000, help="dbsweep: keyframes in the database")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the keypoints, descriptors and matches the value path returned in its "
+                    "last timed step (a fixed sample of %d frames) as DIR/<name>.npy" % DUMP_FRAMES)
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "stream" or args.impl != "orbfe"):
+        ap.error("--dump-outputs writes the results of the stream workload of --impl orbfe")
     if args.workload != "stream" and args.impl == "orbfe":
         sys.path.insert(0, os.path.join(ROOT, "tools"))
         import multi_gpu
@@ -435,6 +442,14 @@ def main():
     host_t = {"extract_call": 0.0, "e2e_extract_call": 0.0, "match_call": 0.0, "views": 0.0, "n": 0}
     ones_u8, zeros_u8 = np.ones(NFEAT, np.uint8), np.zeros(NFEAT, np.uint8)
     checks = {"device": None, "e2e": None}    # last finished sub-step of each path, for the oracle cross-check
+    # --dump-outputs: the sampled frames' results, filled while the last timed step finishes its batches
+    dump_frames = np.sort(np.random.default_rng(0).choice(args.frames, min(args.frames, DUMP_FRAMES), replace=False))
+    dump = {"keypoints": np.zeros((len(dump_frames), NFEAT, 7), np.float32),
+            "descriptors": np.zeros((len(dump_frames), NFEAT, 32), np.float32),
+            "keypoint_counts": np.full(len(dump_frames), -1, np.float32),
+            "matches": np.zeros((len(dump_frames), NFEAT), np.float32),
+            "match_counts": np.zeros(len(dump_frames), np.float32),
+            "frame_index": dump_frames.astype(np.float32)} if args.dump_outputs and rank == 0 else None
 
     Tcws_arr = np.ascontiguousarray(np.stack(Tcws).reshape(args.frames, 12), np.float32)
     ones_ptr, zeros_ptr = np.uint64(ones_u8.ctypes.data), np.uint64(zeros_u8.ctypes.data)
@@ -508,7 +523,7 @@ def main():
     d_last = torch.tensor([B] + list(range(0, B - 1)), dtype=torch.int32, device=dev)
     stream_m = torch.cuda.Stream(device=dev, priority=-1)   # the short matcher kernel goes first when SMs free up
     stream_b = stream_m
-    dev_state = {"step": 0}
+    dev_state = {"step": 0, "capture_from": None}
 
     def enqueue_device_step():
         st = dev_state["step"]
@@ -540,6 +555,7 @@ def main():
             S["h_mp"].copy_(S["mp"], non_blocking=True)
             S["ev_done"].record(stream_m)
         S["sb"] = sb
+        S["capture"] = dump is not None and dev_state["capture_from"] is not None and st >= dev_state["capture_from"]
         launches[0] += ex.last_launches() + 1
         dev_state["step"] = st + 1
         return S
@@ -548,10 +564,30 @@ def main():
         S["ev_done"].synchronize()
         kp_total[0] += int(S["h_cnt"].numpy().sum())
         checks["device"] = S
+        if S["capture"]:
+            capture_batch(S)
         return int(S["h_nm"].numpy().sum())
 
-    def run_device(steps):
+    def capture_batch(S):
+        """--dump-outputs: the sampled frames of this batch, as a caller of the value path receives them (rows past a frame's
+        keypoint count are not part of its result and stay zero)"""
+        lo = S["sb"] * B
+        kd = S["h_kps"].numpy().view(fe.KP_DTYPE).reshape(B, NFEAT)
+        for j in np.flatnonzero((dump_frames >= lo) & (dump_frames < lo + B)):
+            i, n = int(dump_frames[j]) - lo, int(S["h_cnt"].numpy()[int(dump_frames[j]) - lo])
+            dump["keypoints"][j] = 0
+            dump["descriptors"][j] = 0
+            for c, name in enumerate(fe.KP_DTYPE.names):
+                dump["keypoints"][j, :n, c] = kd[i, :n][name]
+            dump["descriptors"][j, :n] = S["h_desc"].numpy()[i, :n]
+            dump["keypoint_counts"][j] = n
+            dump["matches"][j] = S["h_mp"].numpy()[i]
+            dump["match_counts"][j] = S["h_nm"].numpy()[i]
+
+    def run_device(steps, capture_last=False):
+        """`steps` steps of SUB batches; with capture_last the batches of the last step fill `dump`"""
         t0 = time.perf_counter()
+        dev_state["capture_from"] = dev_state["step"] + (steps - 1) * SUB if capture_last else None
         nm, pending = 0, None
         for _ in range(steps * SUB):
             S = enqueue_device_step()
@@ -700,7 +736,7 @@ def main():
     stage_n[0] = 0
 
     sampler.t_begin = time.perf_counter()
-    r_dev = timed(run_device, args.steps)
+    r_dev = timed(lambda steps: run_device(steps, capture_last=dump is not None), args.steps)
     stages = {k: v / max(stage_cnt.get(k, 1), 1) * SUB for k, v in stage_acc.items()}   # ms per step (= SUB library calls)
     if rank == 0 and stage_cnt and min(stage_cnt.values()) != args.steps * SUB:
         sys.stderr.write("bench: stage intervals read back for %s of %d batches\n" % (sorted(set(stage_cnt.values())), args.steps * SUB))
@@ -847,6 +883,11 @@ def main():
                 "roofline": roof, "clocks": clocks}
         if not args.no_cpu_baseline:
             line["cpu_baseline"], _ = cpu_baseline_dict(frames_np, shifts, 1, True)
+        if dump is not None:
+            assert (dump["keypoint_counts"] >= 0).all(), "--dump-outputs: a sampled frame was not produced by the last step"
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line))
     if drv["d"]:
         drv["d"].close()

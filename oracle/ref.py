@@ -30,6 +30,23 @@ def build(force=False):
     return os.path.join(_DIR, "libref_orbslam.so")
 
 
+def shim_lib():
+    """oracle/libref_shim.so: the stand-in cv:: layer of ref_shim/ on its own (no reference source needed), with the
+    ref_shim_gemm / ref_shim_norm self-test hooks."""
+    if "shim" not in _libs:
+        from . import build as build_oracle
+        build_oracle()
+        subprocess.check_call(["make", "-C", _HERE, "-s", "shim"], env={**os.environ, "CC": "gcc", "CXX": "g++"})
+        L = C.CDLL(os.path.join(_HERE, "libref_shim.so"), mode=os.RTLD_NOW | os.RTLD_LOCAL)
+        L.ref_shim_gemm.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_double,
+                                    C.c_int, C.c_void_p]
+        L.ref_shim_gemm.restype = None
+        L.ref_shim_norm.argtypes = [C.c_void_p, C.c_int]
+        L.ref_shim_norm.restype = C.c_double
+        _libs["shim"] = L
+    return _libs["shim"]
+
+
 def available(which="ref"):
     return os.path.exists(os.path.join(_DIR, "lib%s_orbslam.so" % which))
 

@@ -354,17 +354,6 @@ int ref_descriptor_distance(const uint8_t *a, const uint8_t *b) {
 
 }  // extern "C"
 
-// ---- shim self-test hook: cv::gemm of the stand-in header, so that tests can pin it to python-cv2's cv2.gemm ---------------
-extern "C" void ref_shim_gemm(const float *A, int ar, int ac, const float *B, int br, int bc, double alpha, const float *Cm, double beta,
-                              int flags, float *out) {
-    cv::Mat a(ar, ac, CV_32F, const_cast<float *>(A)), b(br, bc, CV_32F, const_cast<float *>(B));
-    const int n = (flags & cv::GEMM_1_T) ? ac : ar, m = (flags & cv::GEMM_2_T) ? br : bc;
-    cv::Mat c = Cm ? cv::Mat(n, m, CV_32F, const_cast<float *>(Cm)) : cv::Mat(), d;
-    cv::gemm(a, b, alpha, c, beta, d, flags);
-    for (int i = 0; i < n; i++) std::memcpy(out + (size_t)i * m, d.ptr(i), sizeof(float) * (size_t)m);
-}
-extern "C" double ref_shim_norm(const float *v, int n) { return cv::norm(cv::Mat(n, 1, CV_32F, const_cast<float *>(v))); }
-
 // =====================================================================================================================
 // KeyFrame-level scenes: keyframes with poses, map points with observations, FeatureVectors -- composed from Python, then
 // the KeyFrame-level matchers (M4, M5, M9-M12) run on them.  Map points and keyframes are addressed by their index in

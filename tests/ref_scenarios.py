@@ -1,11 +1,15 @@
 """One scripted SLAM scene -- two keyframes with poses, map points with observations, FeatureVectors -- run through every
 ORBmatcher method of one build of the reference's map model (oracle/ref.py: "ref" = the reference's own ORBmatcher.cc,
 "facade" = orb_slam_b200/host/ORBmatcher.cc over liborbfe.so, both next to the reference's unmodified Frame.cc /
-KeyFrame.cc / MapPoint.cc).  Returns plain arrays so that two builds, or a build and the oracle, can be compared."""
+KeyFrame.cc / MapPoint.cc).  Returns plain arrays so that two builds, or a build and the oracle, can be compared.  What the
+"ref" build returns is stored in tests/golden/ref_scene.npz (tests/ref_golden.py): run_ref() and features() read it."""
 import numpy as np
 
 from oracle import ref as R
 from orb_slam_b200.synth import textured_frame, shifted_frame
+from ref_golden import Golden, extraction
+
+GOLDEN = Golden("ref_scene")
 
 W, H = 640, 480
 FX = FY = 500.0
@@ -56,8 +60,14 @@ def features():
     if _FEATS is None:
         a = textured_frame(W, H, seed=21)
         b = shifted_frame(a, SHIFT[0], SHIFT[1], seed=1)
-        _FEATS = [R.extract(im, 1000, 1.2, 8, 1, 20) for im in (a, b)]
+        _FEATS = [extraction(GOLDEN, "features%d" % i, im, 1000, 1.2, 8, 1, 20, lambda: R.extract(im, 1000, 1.2, 8, 1, 20))
+                  for i, im in enumerate((a, b))]
     return _FEATS
+
+
+def run_ref():
+    """run("ref"), as stored."""
+    return GOLDEN("run_ref", lambda: run("ref"))
 
 
 def run(which):

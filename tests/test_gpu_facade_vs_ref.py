@@ -2,24 +2,27 @@
 DBoW2 are compiled twice (oracle/Makefile `make ref`) -- once with the reference's own ORBextractor.cc / ORBmatcher.cc, once with
 this repo's include/ORBextractor.h, include/ORBmatcher.h and orb_slam_b200/host/*.cc over liborbfe.so (CUDA) in their place --
 and the same scripted scene (tests/ref_scenarios.py) is run through both: every ORBmatcher method must return the same
-matches, and after Fuse the same map (keyframe slots, bad flags, observations).  Needs a GPU for the facade build."""
-import os
+matches, and after Fuse the same map (keyframe slots, bad flags, observations).  Needs a GPU for the facade build.
 
+The reference build's results are stored (tests/golden/ref_*.npz, see tests/ref_golden.py); the facade build compiles the
+reference's Frame.cc / KeyFrame.cc / MapPoint.cc, so these tests run only where that build exists (oracle/Makefile `make ref`
+with the reference sources at ORB_REFERENCE_ROOT) and skip elsewhere."""
 import numpy as np
 import pytest
 
 import oracle as O
 from oracle import ref as R
+from ref_golden import Golden, extraction
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not (R.available("facade") and R.available("ref")),
-                                 reason="oracle/_ref/*.so are built from /root/reference (absent here) and no prebuilt libraries travel with this checkout")]
+              pytest.mark.skipif(not R.available("facade"),
+                                 reason="oracle/_ref/libfacade_orbslam.so is built from the reference sources, which this checkout does not contain")]
 
 
 @pytest.fixture(scope="module")
 def both(gpu_required):
     import ref_scenarios as RS
-    return RS, RS.run("ref"), RS.run("facade")
+    return RS, RS.run_ref(), RS.run("facade")
 
 
 @pytest.mark.parametrize("key", ["m4_a", "m4_b", "m4_c", "m5_a", "m5_b", "m9_kf_f_a", "m9_kf_f_b", "m9_kf_kf_a", "m9_kf_kf_b", "m10_a",
@@ -34,9 +37,8 @@ def test_frame_level_methods_equal_the_reference(gpu_required):
     """M2, M3, M6, M7, M8 through real Frame objects, both builds."""
     import ref_scenarios as RS
     (k1, d1), (k2, d2) = RS.features()
-    rng = np.random.default_rng(9)
-    res = {}
-    for which in ("ref", "facade"):
+
+    def frame_level(which):
         rng = np.random.default_rng(9)
         f1 = R.RefFrame.from_arrays(k1, d1, RS.W, RS.H, RS.FX, RS.FY, RS.CX, RS.CY, which=which)
         f2 = R.RefFrame.from_arrays(k2, d2, RS.W, RS.H, RS.FX, RS.FY, RS.CX, RS.CY, which=which)
@@ -57,9 +59,10 @@ def test_frame_level_methods_equal_the_reference(gpu_required):
         r["m3"] = [R.search_local_points(f2, in_view, proj, k1["octave"].astype(np.int32), vcos, d1, th, 0.8, f_mp=pre) for th in (3.0, 1.0)]
         r["m6"] = [R.search_by_projection_f1f2(f1, f2, has, RS.backproject(k1), T, win, 0.9, f2_mp=pre) for win in (10, 25)]
         r["m1"] = R.descriptor_distance(d1[3], d2[7], which=which)
-        res[which] = r
         f1.close()
         f2.close()
+        return r
+    res = {"ref": RS.GOLDEN("frame_level", lambda: frame_level("ref")), "facade": frame_level("facade")}
     for key in res["ref"]:
         assert RS.same(res["ref"][key], res["facade"][key]), key
     assert res["ref"]["m2"][0][0] > 300 and res["ref"]["m8"][0] > 20
@@ -72,7 +75,8 @@ def test_extractor_facade_against_the_reference_sources(gpu_required):
     import ref_scenarios as RS
     from orb_slam_b200.synth import textured_frame
     img = textured_frame(640, 480, seed=21)
-    rk, rd = R.extract(img, 1000, 1.2, 8, 1, 20, which="ref")
+    rk, rd = extraction(Golden("ref_extract"), "extract_640_480_1000_8_1_21", img, 1000, 1.2, 8, 1, 20,
+                        lambda: R.extract(img, 1000, 1.2, 8, 1, 20, which="ref"))
     fk, fd = R.extract(img, 1000, 1.2, 8, 1, 20, which="facade")
     assert len(rk) == len(fk) == 1000
     rc, ok, od, _ = O.extract(O.make_params(1000, 1.2, 8, 1, 20), img)     # the facade == the oracle's canonical mode, bit for bit
